@@ -22,6 +22,12 @@ synthetic data.  Prints ONE JSON line:
   cpu_baseline the reference algorithm's CPU step (oracle port) on the host cores
 `--impl reference` times the reference algorithm's CPU path on all host cores (oracle
 port: the reference needs TensorFlow, which cannot be installed here).
+
+`--dump-outputs DIR` writes what the last timed step computed to DIR/<name>.npy (float32,
+or float64 for float64 arrays): for configs 2-4 the loss, per-list losses, scores, d loss /
+d scores, the flat scorer gradient and the updated parameters; for config 5 the loss,
+per-list losses and d loss / d scores of every sweep row.  Inputs and initial parameters
+are seeded, so two builds run with the same arguments can be compared file by file.
 """
 import argparse
 import json
@@ -30,6 +36,8 @@ import subprocess
 import sys
 import threading
 import time
+
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from unchanged
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -96,6 +104,25 @@ def load_peaks():
             'source': 'measured'}
   return {'hbm_gbs': 6650.0, 'bf16_tflops': 1590.0,
           'bf16_tflops_sustained': 1400.0, 'source': 'fallback'}
+
+
+DUMP_MAX_ELEMS = 1 << 18   # keeps a config-5 dump (12 sweep rows) near 15 MB
+
+
+def dump_outputs(out_dir, arrays):
+  """Writes every tensor of `arrays` (name -> tensor) to out_dir/<name>.npy, float64 tensors
+  as float64 and all others as float32.  A tensor of more than DUMP_MAX_ELEMS elements is
+  written as its flattened elements at DUMP_MAX_ELEMS sorted indices drawn with a fixed
+  seed, the same indices for every run of the same shape."""
+  import numpy as np
+  os.makedirs(out_dir, exist_ok=True)
+  for name, t in arrays.items():
+    t = t.detach()
+    t = t.double() if t.dtype == torch.float64 else t.float()
+    if t.numel() > DUMP_MAX_ELEMS:
+      idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))
+      t = t.reshape(-1)[idx[:DUMP_MAX_ELEMS].sort().values.to(t.device)]
+    np.save(os.path.join(out_dir, name + '.npy'), t.cpu().numpy())
 
 
 class ClockSampler(threading.Thread):
@@ -400,6 +427,10 @@ def run_gpu(args):
   launches = _C.lib.tfr_launch_count() - launches0
   ms_total = ev0.elapsed_time(ev1)
   sampler.mark(t_val0, time.perf_counter())
+  if args.dump_outputs and rank == 0:   # before the phase and e2e runs step the trainer on
+    dump_outputs(args.dump_outputs, {
+        'loss': loss, 'per_list_loss': trainer.per_list[0], 'scores': trainer.scores,
+        'dscores': trainer.dscores, 'grads': trainer.grads, 'params': tower.flat})
   t = torch.tensor([ms_total], dtype=torch.float64, device=dev)
   if world > 1:
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -699,6 +730,11 @@ def run_sweep(args):
         torch.cuda.synchronize()
       sampler.mark(t0, time.perf_counter())
       launches += _C.lib.tfr_launch_count() - l0
+      if args.dump_outputs and rank == 0:
+        tag = '%s_N%d_' % (lam_name, n)
+        dump_outputs(args.dump_outputs, {tag + 'loss': total2[0],
+                                         tag + 'per_list_loss': per_list[0],
+                                         tag + 'dscores': grad})
       t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
       if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -762,7 +798,13 @@ def main():
   ap.add_argument('--cpu-sample-lists', type=int, default=0)
   ap.add_argument('--cpu-steps', type=int, default=3)
   ap.add_argument('--no-cpu-baseline', action='store_true')
+  ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                  help='write the outputs of the last timed step to DIR/<name>.npy')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl == 'reference':
+    ap.error('--dump-outputs dumps the CUDA path: use it with --impl b200')
   args.warmup = max(args.warmup, 3)
   # The contract is ONE JSON line on stdout.  Libraries print banners there (e.g.
   # "NCCL version ..." at communicator creation), so everything but the final line is
