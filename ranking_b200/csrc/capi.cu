@@ -116,19 +116,7 @@ int make_mlp_plan(const tfr_mlp_cfg* cfg, int M, MlpPlan* p) {
   }
   // Row splits of the dW GEMMs / bias partials: about one per SM, so that the
   // persistent GEMM's tile list (m_tiles x splits) divides evenly over the SMs.
-  {
-    static int num_sms = 0;
-    if (num_sms == 0) {
-      int dev = 0;
-      if (cudaGetDevice(&dev) != cudaSuccess ||
-          cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess ||
-          num_sms <= 0)
-        num_sms = 148;   // B200 (also the answer on a CPU-only build box)
-    }
-    const int per = (M + num_sms - 1) / num_sms;
-    p->rows_per_split = per < 256 ? 256 : ((per + 127) / 128) * 128;
-    p->splits = M > 0 ? (M + p->rows_per_split - 1) / p->rows_per_split : 1;
-  }
+  p->splits = dw_row_splits(M, &p->rows_per_split);
   p->partial_stride = align_up(max_wb, 64);
   p->partial_off = w;
   w += (size_t)p->splits * p->partial_stride;
@@ -198,12 +186,6 @@ extern "C" size_t tfr_mlp_workspace_bytes(const tfr_mlp_cfg* cfg, int M) {
   MlpPlan p;
   if (make_mlp_plan(cfg, M, &p)) return 0;
   return p.ws_floats * sizeof(float) + 256;
-}
-
-static float* ws_base(void* workspace) {
-  uintptr_t a = reinterpret_cast<uintptr_t>(workspace);
-  a = (a + 255) & ~(uintptr_t)255;
-  return reinterpret_cast<float*>(a);
 }
 
 extern "C" int tfr_mlp_fwd(const void* Xv, int M, const tfr_mlp_cfg* cfg,

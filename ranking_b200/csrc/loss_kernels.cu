@@ -8,8 +8,6 @@
 // ends, so no scatter/atomic is needed and results are deterministic.
 #include <math_constants.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "loss_common.cuh"
 
@@ -921,9 +919,8 @@ extern "C" int tfr_pairwise_loss_fwd_bwd(const float* scores, const float* label
   const size_t smem = list_smem_bytes(N);
   cudaStream_t st = (cudaStream_t)stream;
   // One phi evaluation per unordered pair (pairwise_tri.cu); the both-ends kernel below
-  // keeps PairwiseMSELoss and N > 1024 (TFR_K1_BOTH_ENDS=1 forces it: A/B measurements).
-  static const bool both_ends = getenv("TFR_K1_BOTH_ENDS") != nullptr;
-  if (phi != TFR_PHI_MSE && N <= 1024 && !both_ends)
+  // keeps PairwiseMSELoss and N > 1024.
+  if (phi != TFR_PHI_MSE && N <= 1024)
     return launch_pairwise_tri(phi, st, scores, labels, item_w, w_per_item, mask, B, N,
                                temperature, lam, grad_scale, grad, row_loss, loss_sum, w_sum,
                                nnz, ranks_out);

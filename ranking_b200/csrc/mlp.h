@@ -5,6 +5,7 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include "tc_gemm.cuh"
 #include "tfr_b200.h"
 
 namespace tfr {
@@ -64,6 +65,14 @@ int mlp_input_bn_bwd(const float* X, int M, const MlpPlan& p, const float* param
 // Returns 0 on success and fills `p`; sets the error string otherwise.
 int make_mlp_plan(const tfr_mlp_cfg* cfg, int M, MlpPlan* p);
 
+// The caller's workspace from its first 256-byte boundary (the *_workspace_bytes queries
+// include the 256 bytes).
+inline float* ws_base(void* workspace) {
+  uintptr_t a = reinterpret_cast<uintptr_t>(workspace);
+  a = (a + 255) & ~(uintptr_t)255;
+  return reinterpret_cast<float*>(a);
+}
+
 int mlp_simt_fwd(const float* X, int M, const MlpPlan& p, const float* params,
                  const uint8_t* mask, float* ws, float* scores, cudaStream_t st);
 int mlp_simt_bwd(const float* X, int M, const MlpPlan& p, const float* params,
@@ -100,6 +109,18 @@ int mlp_tc_fwd_from(int first_layer, const float* X, int M, const MlpPlan& p,
 int mlp_tc_bwd_until(int stop_layer, MlpBwdTail* tail, const float* X, int M, const MlpPlan& p,
                      const float* params, const float* dscores, const uint8_t* mask,
                      float* ws, float* grads, int passes, cudaStream_t st);
+
+// Dense layers as 3xTF32 / TF32 GEMMs (mlp_tc.cu), shared by the tower and the groupwise fold.
+// Forward of Dense d over rows k0 .. k0 + K - 1 of its kernel W [dims[d], dims[d + 1]]:
+// C[M, dims[d + 1]] = A[M, K] W[k0 : k0 + K, :].  C and the epilogue are the caller's.
+tc::GemmDesc dense_fwd_gemm(const MlpPlan& p, int d, int k0, int K, const float* A, int M,
+                            const float* params, const float* ws, int passes);
+// dW[Kin, Nout] = A^T dZ over `rows` rows (A [rows, Kin], dZ [rows, Nout], row-major), as
+// `splits` row-range partials C + z * split_stride, each [Kin, Nout] row-major.
+tc::GemmDesc dense_dw_gemm(const float* A, int Kin, const float* dZ, int Nout, int rows,
+                           int passes, float* C, int splits, size_t split_stride);
+// Row ranges the dW GEMMs over `rows` rows are split into (about one per SM).
+int dw_row_splits(int rows, int* rows_per_split);
 
 // pieces of the CUDA-core path reused by the tensor-core path
 int mlp_out_layer_fwd(const float* H, int M, int K, int O, const float* W, const float* bias,

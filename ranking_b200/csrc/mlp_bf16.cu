@@ -20,6 +20,7 @@
 #include "common.cuh"
 #include "mlp.h"
 #include "tc_gemm_bf16.cuh"
+#include "tc_host.h"
 
 namespace tfr {
 
@@ -392,7 +393,7 @@ int mlp_bf16_fwd(const void* X, int M, const MlpPlan& p, const float* params,
   }
   const int K = p.dims[L], O = p.dims[L + 1];
   if (K <= kFastK && O <= kFastO) {
-    const int nb = (M + 31) / 32 < 148 * 8 ? (M + 31) / 32 : 148 * 8;   // 32 rows per block pass
+    const int nb = (M + 31) / 32 < num_sms() * 8 ? (M + 31) / 32 : num_sms() * 8;   // 32 rows a pass
     const uint4* H8 = reinterpret_cast<const uint4*>(in);
     const float* Wl = params + p.w_off[L];
     const float* bl = params + p.b_off[L];
@@ -406,7 +407,7 @@ int mlp_bf16_fwd(const void* X, int M, const MlpPlan& p, const float* params,
     TFR_LAUNCH_OK();
     return TFR_OK;
   }
-  const int blocks = (M + 7) / 8 < 148 * 16 ? (M + 7) / 8 : 148 * 16;
+  const int blocks = (M + 7) / 8 < num_sms() * 16 ? (M + 7) / 8 : num_sms() * 16;
   out_fwd_bf16_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<const __nv_bfloat162*>(in), M,
                                               K / 2, O, params + p.w_off[L], params + p.b_off[L],
                                               mask, scores);

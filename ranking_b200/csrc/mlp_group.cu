@@ -22,6 +22,7 @@
 #include "common.cuh"
 #include "mlp.h"
 #include "tc_gemm.cuh"
+#include "tc_host.h"
 
 namespace tfr {
 
@@ -331,7 +332,7 @@ extern "C" int tfr_circular_pad_gather(const void* x, const uint8_t* is_valid, i
   const int row_vecs = row_bytes / 16;
   const size_t total = (size_t)B * N * row_vecs;
   size_t blocks = (total + 255) / 256;
-  if (blocks > 148 * 16) blocks = 148 * 16;
+  if (blocks > (size_t)num_sms() * 16) blocks = (size_t)num_sms() * 16;
   gather_rows_kernel<<<(unsigned)blocks, 256, 0, st>>>(static_cast<const uint4*>(x), idx_out, N,
                                                       row_vecs, total, static_cast<uint4*>(out));
   TFR_LAUNCH_OK();
@@ -346,12 +347,6 @@ extern "C" size_t tfr_group_mlp_workspace_bytes(const tfr_mlp_cfg* cfg, int B, i
   return (p.ws_floats + group_extra_floats(B, N, G, gs, p.dims[1])) * sizeof(float) + 256;
 }
 
-static float* group_ws_base(void* workspace) {
-  uintptr_t a = reinterpret_cast<uintptr_t>(workspace);
-  a = (a + 255) & ~(uintptr_t)255;
-  return reinterpret_cast<float*>(a);
-}
-
 extern "C" int tfr_group_mlp_fwd(const float* X, int B, int N, int G, int gs, const int32_t* idx,
                                  const uint8_t* gmask, const tfr_mlp_cfg* cfg,
                                  const float* params, void* workspace, float* logits_out,
@@ -362,7 +357,7 @@ extern "C" int tfr_group_mlp_fwd(const float* X, int B, int N, int G, int gs, co
   TFR_REQUIRE(X && idx && gmask && params && workspace && logits_out, "NULL argument");
   cudaStream_t st = (cudaStream_t)stream;
   const int passes = precision == TFR_PREC_TF32X3 ? 3 : 1;
-  float* ws = group_ws_base(workspace);
+  float* ws = ws_base(workspace);
   const int D = p.dims[0] / gs, H = p.dims[1], M = B * G, S = G / N;
   const size_t bn = (size_t)B * N;
   GroupWs gw = carve_group(ws + p.ws_floats, B, N, G, gs, H);
@@ -380,26 +375,12 @@ extern "C" int tfr_group_mlp_fwd(const float* X, int B, int N, int G, int gs, co
   }
   rc = mlp_tc_split_params(p, params, ws, passes, st);
   if (rc) return rc;
-  const float* whi = passes == 3 ? ws + p.whi_off : params;
-  const float* wlo = passes == 3 ? ws + p.wlo_off : nullptr;
-  // P_j = X W_1^(j): the first Dense layer on the ungathered [B * N, D] matrix
+  // P_j = X W_1^(j): the first Dense layer on the ungathered [B * N, D] matrix, with slot j's
+  // rows j D .. (j + 1) D of W_1
   for (int j = 0; j < gs; ++j) {
-    tc::GemmDesc g{};
-    g.A = X; g.lda = D;
-    if (passes == 3) {
-      // slot j of W_1^T [H, gs * D] (pre-split transposes, K-major): columns j D .. (j + 1) D
-      g.B = ws + p.wthi_off + p.w_off[0] + (size_t)j * D; g.ldb = gs * D;
-      g.B_lo = ws + p.wtlo_off + p.w_off[0] + (size_t)j * D;
-      g.b_mn = 0;
-    } else {
-      g.B = whi + p.w_off[0] + (size_t)j * D * H; g.ldb = H;
-      g.B_lo = nullptr;
-      g.b_mn = 1;
-    }
+    tc::GemmDesc g = dense_fwd_gemm(p, 0, j * D, D, X, (int)bn, params, ws, passes);
     g.C = gw.P + (size_t)j * gw.p_stride; g.ldc = H;
-    g.GM = (int)bn; g.GN = H; g.GK = D;
-    g.a_mn = 0; g.passes = passes; g.split_b = 0;
-    g.epi = tc::EPI_STORE; g.act = TFR_ACT_NONE; g.splits = 1;
+    g.epi = tc::EPI_STORE; g.act = TFR_ACT_NONE;
     rc = tc::gemm(g, st);
     if (rc) return rc;
   }
@@ -427,7 +408,7 @@ extern "C" int tfr_group_mlp_check(const tfr_mlp_cfg* cfg, int B, int N, int G, 
   MlpPlan p;
   int rc = make_mlp_plan(cfg, B * G, &p);
   if (rc) return rc;
-  float* ws = group_ws_base(workspace);
+  float* ws = ws_base(workspace);
   GroupWs gw = carve_group(ws + p.ws_floats, B, N, G, gs, p.dims[1]);
   int flag = 0;
   TFR_CUDA_OK(cudaMemcpyAsync(&flag, gw.dup, sizeof(int), cudaMemcpyDeviceToHost,
@@ -449,7 +430,7 @@ extern "C" int tfr_group_mlp_bwd(const float* X, int B, int N, int G, int gs, co
   TFR_REQUIRE(X && idx && gmask && params && workspace && dlogits && grads, "NULL argument");
   cudaStream_t st = (cudaStream_t)stream;
   const int passes = precision == TFR_PREC_TF32X3 ? 3 : 1;
-  float* ws = group_ws_base(workspace);
+  float* ws = ws_base(workspace);
   const int D = p.dims[0] / gs, H = p.dims[1], M = B * G, S = G / N;
   const size_t bn = (size_t)B * N;
   GroupWs gw = carve_group(ws + p.ws_floats, B, N, G, gs, H);
@@ -464,9 +445,8 @@ extern "C" int tfr_group_mlp_bwd(const float* X, int B, int N, int G, int gs, co
   rc = mlp_tc_bwd_until(1, &tail, nullptr, M, p, params, gw.gscore, nullptr, ws, grads, passes, st);
   if (rc) return rc;
   // first layer: dP_j by the inverse index, dW_1^(j) = X^T dP_j (rows split over CTAs)
-  const int per = (int)((bn + 147) / 148);
-  const int rows_per = per < 256 ? 256 : ((per + 127) / 128) * 128;
-  int splits = (int)((bn + rows_per - 1) / rows_per);
+  int rows_per = 0;
+  int splits = dw_row_splits((int)bn, &rows_per);
   if (splits > p.splits) splits = p.splits;
   for (int j = 0; j < gs; ++j) {
     float* dP = gw.P + (size_t)j * gw.p_stride;
@@ -474,30 +454,8 @@ extern "C" int tfr_group_mlp_bwd(const float* X, int B, int N, int G, int gs, co
     group_gather_bwd_kernel<<<(unsigned)((t + 255) / 256), 256, 0, st>>>(tail.dz, gw.inv, S, B, N,
                                                                          G, gs, j, H, dP);
     TFR_LAUNCH_OK();
-    // dW^(j)^T [H, D] = dP_j^T X, stored transposed (the orientation of mlp_tc_bwd when the
-    // output width is the larger side is decided the same way: fewer UMMA tiles)
-    auto cost = [](int gm, int gn) {
-      const int n16 = (gn + 15) / 16 * 16;
-      const int ntiles = (n16 + 255) / 256;
-      const int n_umma = n16 < 256 ? n16 : 256;
-      const long long mmas = (long long)((gm + 127) / 128) * ntiles;
-      return mmas * (1 << 20) + mmas * (16384 + 128 * n_umma);
-    };
-    const bool swapped = cost(H, D) < cost(D, H);
-    tc::GemmDesc g{};
-    if (!swapped) {
-      g.A = X; g.lda = D; g.B = dP; g.ldb = H;
-      g.GM = D; g.GN = H; g.store_transposed = 0;
-    } else {
-      g.A = dP; g.lda = H; g.B = X; g.ldb = D;
-      g.GM = H; g.GN = D; g.store_transposed = 1;
-    }
-    g.C = ws + p.partial_off; g.ldc = H;
-    g.GK = (int)bn;
-    g.a_mn = 1; g.b_mn = 1; g.passes = passes; g.split_b = 1;
-    g.epi = tc::EPI_STORE;
-    g.splits = splits; g.split_stride = p.partial_stride;
-    rc = tc::gemm(g, st);
+    rc = tc::gemm(dense_dw_gemm(X, D, dP, H, (int)bn, passes, ws + p.partial_off, splits,
+                                p.partial_stride), st);
     if (rc) return rc;
     const bool last = j == gs - 1;   // the bias gradient follows the last slot's block
     rc = mlp_reduce2(ws + p.partial_off, splits, p.partial_stride, (size_t)D * H,

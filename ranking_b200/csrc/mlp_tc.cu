@@ -11,6 +11,7 @@
 #include "common.cuh"
 #include "mlp.h"
 #include "tc_gemm.cuh"
+#include "tc_host.h"
 
 namespace tfr {
 
@@ -83,6 +84,73 @@ static int split_params(const MlpPlan& p, const float* params, float* ws, int pa
   return TFR_OK;
 }
 
+tc::GemmDesc dense_fwd_gemm(const MlpPlan& p, int d, int k0, int K, const float* A, int M,
+                            const float* params, const float* ws, int passes) {
+  const int N = p.dims[d + 1];
+  tc::GemmDesc g{};
+  g.A = A; g.lda = K;
+  if (passes == 3) {   // W^T [out, in], pre-split: K-major
+    g.B = ws + p.wthi_off + p.w_off[d] + k0; g.ldb = p.dims[d];
+    g.B_lo = ws + p.wtlo_off + p.w_off[d] + k0;
+    g.b_mn = 0;
+  } else {             // single-pass TF32 reads the fp32 kernel [in, out] as is: MN-major
+    g.B = params + p.w_off[d] + (size_t)k0 * N; g.ldb = N;
+    g.B_lo = nullptr;
+    g.b_mn = 1;
+  }
+  g.GM = M; g.GN = N; g.GK = K;
+  g.a_mn = 0; g.passes = passes; g.split_b = 0;
+  g.splits = 1; g.split_stride = 0;
+  return g;
+}
+
+tc::GemmDesc dense_dw_gemm(const float* A, int Kin, const float* dZ, int Nout, int rows,
+                           int passes, float* C, int splits, size_t split_stride) {
+  // dW[Kin, Nout] = A^T dZ in one of two orientations:
+  //   direct : GM = Kin (tiles of 128), GN = Nout
+  //   swapped: GM = Nout,               GN = Kin, stored transposed
+  // Cost of one 32-row k block (tools/mma_rate.cu: a 128 x N x 8 TF32 MMA takes N / 2
+  // cycles; profiles/r02_tc_gemm_wait_cycles.txt: the dW GEMMs are bound by shared-memory
+  // traffic, 128 B / cycle): per 128-row block of the M side the stage is written by TMA,
+  // read by the splitters (the M side goes to tensor memory), the N side is rewritten as
+  // hi / lo and read by 12 MMAs.  Fewer than 3 pipeline stages expose the load latency.
+  auto cost = [](int gm, int gn) {
+    const int n16 = (gn + 15) / 16 * 16;
+    const int ntiles = (n16 + 255) / 256;
+    const int n_umma = n16 < 256 ? n16 : 256;
+    const long long tiles = (long long)((gm + 127) / 128) * ntiles;
+    const long long mma = tiles * 12 * (n_umma / 2);
+    const long long smem = tiles * (32768 + 896LL * n_umma) / 128;
+    const long long stage = 16384 + 256LL * n_umma;
+    long long c = mma > smem ? mma : smem;
+    if (200 * 1024 / stage < 3) c = c * 3 / 2;
+    return c;
+  };
+  const bool swapped = cost(Nout, Kin) < cost(Kin, Nout);
+  tc::GemmDesc g{};
+  if (!swapped) {
+    g.A = A; g.lda = Kin; g.B = dZ; g.ldb = Nout;
+    g.GM = Kin; g.GN = Nout; g.store_transposed = 0;
+  } else {
+    g.A = dZ; g.lda = Nout; g.B = A; g.ldb = Kin;
+    g.GM = Nout; g.GN = Kin; g.store_transposed = 1;
+  }
+  g.B_lo = nullptr;
+  g.C = C; g.ldc = Nout;
+  g.GK = rows;
+  g.a_mn = 1; g.b_mn = 1; g.passes = passes; g.split_b = 1;
+  g.epi = tc::EPI_STORE;
+  g.splits = splits; g.split_stride = split_stride;
+  return g;
+}
+
+int dw_row_splits(int rows, int* rows_per_split) {
+  const int sms = num_sms();
+  const int per = (rows + sms - 1) / sms;
+  *rows_per_split = per < 256 ? 256 : ((per + 127) / 128) * 128;
+  return rows > 0 ? (rows + *rows_per_split - 1) / *rows_per_split : 1;
+}
+
 int mlp_tc_split_params(const MlpPlan& p, const float* params, float* ws, int passes,
                         cudaStream_t st) {
   int rc = check_dims(p);
@@ -107,8 +175,6 @@ int mlp_tc_fwd_from(int first_layer, const float* X, int M, const MlpPlan& p,
     if (rc) return rc;
   }
   const int L = p.n_dense - 1;
-  const float* whi = passes == 3 ? ws + p.whi_off : params;
-  const float* wlo = passes == 3 ? ws + p.wlo_off : nullptr;
   const float* in = X;
   if (p.input_bn && first_layer == 0) {
     rc = mlp_input_bn_fwd(X, M, p, params, ws, st);
@@ -116,23 +182,10 @@ int mlp_tc_fwd_from(int first_layer, const float* X, int M, const MlpPlan& p,
     in = ws + p.xin_off;
   }
   for (int d = first_layer; d < L; ++d) {
-    tc::GemmDesc g{};
-    g.A = in; g.lda = p.dims[d];
-    if (passes == 3) {   // W^T [out, in], pre-split: K-major
-      g.B = ws + p.wthi_off + p.w_off[d]; g.ldb = p.dims[d];
-      g.B_lo = ws + p.wtlo_off + p.w_off[d];
-      g.b_mn = 0;
-    } else {             // single-pass TF32 reads the fp32 kernel [in, out] as is: MN-major
-      g.B = whi + p.w_off[d]; g.ldb = p.dims[d + 1];
-      g.B_lo = nullptr;
-      g.b_mn = 1;
-    }
+    tc::GemmDesc g = dense_fwd_gemm(p, d, 0, p.dims[d], in, M, params, ws, passes);
     g.C = ws + (p.use_bn ? p.xhat_off[d] : p.act_off[d]); g.ldc = p.dims[d + 1];
-    g.GM = M; g.GN = p.dims[d + 1]; g.GK = p.dims[d];
-    g.a_mn = 0; g.passes = passes; g.split_b = 0;
     g.epi = tc::EPI_BIAS_ACT; g.bias = params + p.b_off[d];
     g.act = p.use_bn ? TFR_ACT_NONE : p.activation;   // BN sits before the activation
-    g.splits = 1; g.split_stride = 0;
     // ReLU sign bits for the backward mask: 1 bit per activation instead of re-reading H
     if (p.activation == TFR_ACT_RELU && !p.post())
       g.mask_bits_out = reinterpret_cast<uint32_t*>(ws + p.bits_off[d]);
@@ -206,45 +259,8 @@ int mlp_tc_bwd_until(int stop_layer, MlpBwdTail* tail, const float* X, int M, co
       bslots = splits;
       bstride = p.tile_stride;
     }
-    {
-      // dW[Kin, Nout] = A^T dZ in one of two orientations:
-      //   direct : GM = Kin (tiles of 128), GN = Nout
-      //   swapped: GM = Nout,               GN = Kin, stored transposed
-      // Cost of one 32-row k block (tools/mma_rate.cu: a 128 x N x 8 TF32 MMA takes N / 2
-      // cycles; profiles/r02_tc_gemm_wait_cycles.txt: the dW GEMMs are bound by shared-memory
-      // traffic, 128 B / cycle): per 128-row block of the M side the stage is written by TMA,
-      // read by the splitters (the M side goes to tensor memory), the N side is rewritten as
-      // hi / lo and read by 12 MMAs.  Fewer than 3 pipeline stages expose the load latency.
-      auto cost = [](int gm, int gn) {
-        const int n16 = (gn + 15) / 16 * 16;
-        const int ntiles = (n16 + 255) / 256;
-        const int n_umma = n16 < 256 ? n16 : 256;
-        const long long tiles = (long long)((gm + 127) / 128) * ntiles;
-        const long long mma = tiles * 12 * (n_umma / 2);
-        const long long smem = tiles * (32768 + 896LL * n_umma) / 128;
-        const long long stage = 16384 + 256LL * n_umma;
-        long long c = mma > smem ? mma : smem;
-        if (200 * 1024 / stage < 3) c = c * 3 / 2;
-        return c;
-      };
-      const bool swapped = cost(Nout, Kin) < cost(Kin, Nout);
-      tc::GemmDesc g{};
-      if (!swapped) {
-        g.A = A; g.lda = Kin; g.B = dz_cur; g.ldb = Nout;
-        g.GM = Kin; g.GN = Nout; g.store_transposed = 0;
-      } else {
-        g.A = dz_cur; g.lda = Nout; g.B = A; g.ldb = Kin;
-        g.GM = Nout; g.GN = Kin; g.store_transposed = 1;
-      }
-      g.B_lo = nullptr;
-      g.C = partial; g.ldc = Nout;
-      g.GK = M;
-      g.a_mn = 1; g.b_mn = 1; g.passes = passes; g.split_b = 1;
-      g.epi = tc::EPI_STORE;
-      g.splits = splits; g.split_stride = pstride;
-      rc = tc::gemm(g, st);
-      if (rc) return rc;
-    }
+    rc = tc::gemm(dense_dw_gemm(A, Kin, dz_cur, Nout, M, passes, partial, splits, pstride), st);
+    if (rc) return rc;
     rc = mlp_reduce2(partial, splits, pstride, (size_t)Kin * Nout, bsrc, bslots, bstride,
                      (size_t)Nout, grads + p.w_off[d], st);
     if (rc) return rc;

@@ -21,10 +21,9 @@
 // tile i+1 and the prologue (barrier init, TMEM allocation) is paid once per SM.
 #include <cuda.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "tc_gemm.cuh"
+#include "tc_host.h"
 #include "tc_ptx.cuh"
 
 namespace tfr {
@@ -38,18 +37,18 @@ constexpr int kThreads = (kEpiWarp0 + kEpiWarps) * 32;   // 576
 constexpr int kEpiSmemBytes = 4 * 32 * 37 * 4;   // fallback stores (4 warps): transpose buffers
 constexpr int kEpiSmemBytes2 = kEpiWarps * 4096; // TMA-store path: one staging tile per warp
 constexpr int BM = 128;       // UMMA M (cta_group::1)
-constexpr int BK = 32;        // fp32 elements per 128-byte swizzle span
+constexpr int BK = 32;        // fp32 elements per 128-byte swizzle span = k of one stage
 constexpr int kATileBytes = BM * BK * 4;   // 16 KB
+constexpr int kBoxBytes = BK * 128;        // one MN-major TMA box: [32 k rows][128 B]
 constexpr int kMaxStages = 4;
+constexpr int kMaxN = 256;    // widest UMMA N: wider outputs are cut into tiles of 256
 
 struct KernelArgs {
   float* C;
   int ldc;
   int GM, GN, GK;
   int n_umma;          // UMMA N of one tile (multiple of 16, <= 256)
-  int bk;              // k extent of one pipeline stage: 32, or 16 when both operands
-                       //   are MN-major (smaller stages -> deeper ring for the dW GEMMs)
-  int a_tile_bytes;    // bytes of one A stage tile (hi part) = 128 * bk * 4
+  int a_tile_bytes;    // bytes of one A stage tile (hi part) = 128 * BK * 4
   int b_tile_bytes;    // bytes of one B stage tile (hi part)
   int stages;
   int epi, act, store_transposed;
@@ -65,16 +64,12 @@ struct KernelArgs {
   long long* dbg;      // optional [gridDim.x][12] wait-cycle counters per warp role
   int vec_ok;          // C / aux / bias / colsum allow 16-byte vector access
   int tma_store;       // row-major unsplit output: epilogue stores 32x32 blocks by TMA
-  int epi_bufs;        // staging tiles per epilogue warp in that mode (1 or 2)
   int epi_smem_bytes;  // bytes of the epilogue staging region
   int colsum_regs;     // column sums kept in registers (single n tile, tma_store)
   int bias_cols;       // floats of the bias copy staged in smem (tma_store + EPI_BIAS_ACT)
   int a_tmem;          // 3xTF32, K-major A: the splitters write A_hi / A_lo to tensor memory
                        //   and the MMAs read A from there (halves the smem operand traffic)
   uint32_t a_col0;     // first TMEM column of the A region: stage s at a_col0 + 64 s
-  int pf_dist;         // k blocks the producer's L2 prefetch runs ahead of its loads (0 = off)
-  int b_resident;      // pairs, pre-split K-major B: this CTA's half of B (hi + lo, every k block)
-                       //   is loaded ONCE and stays in shared memory; stages hold A only
   uint32_t acc_bufs;   // accumulator buffers in TMEM (2: epilogue overlaps the next tile;
                        //   1: long split-K tiles whose A stages need the columns)
   uint32_t tmem_alloc_cols;   // power of two >= 2 * tmem_cols (+ 64 * stages with a_tmem)
@@ -108,14 +103,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   const int kACopies = (PASSES == 3 && !args.a_tmem) ? 2 : 1;
   constexpr int kBCopies = PASSES == 3 ? 2 : 1;
   const int a_bytes = args.a_tile_bytes * kACopies;
-  const bool b_res = CG2 && !B_MN && !SPLIT_B && PASSES == 3 && args.b_resident;
-  const int stage_bytes = a_bytes + (b_res ? 0 : args.b_tile_bytes * kBCopies);
+  const int stage_bytes = a_bytes + args.b_tile_bytes * kBCopies;
   const int S = args.stages;
-  // resident B (b_res): [k block][hi | lo] right after the ring
-  unsigned char* bres = smem + static_cast<size_t>(S) * stage_bytes;
-  const int nkb_all = (args.GK + args.bk - 1) / args.bk;
-  unsigned char* epi_smem =
-      bres + (b_res ? static_cast<size_t>(nkb_all) * 2 * args.b_tile_bytes : 0);   // 4 x [32][33] floats
+  unsigned char* epi_smem = smem + static_cast<size_t>(S) * stage_bytes;   // 4 x [32][33] floats
   float* cacc_base = reinterpret_cast<float*>(epi_smem + args.epi_smem_bytes);   // [4][colsum_cols]
   float* sbias = cacc_base + kEpiWarps * args.colsum_cols;                       // [bias_cols]
   uint64_t* bars = reinterpret_cast<uint64_t*>(
@@ -127,12 +117,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
   uint64_t* acc_full = bars + 3 * kMaxStages;    // [2] accumulator buffer complete
   uint64_t* acc_empty = bars + 3 * kMaxStages + 2;   // [2] accumulator buffer drained
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * kMaxStages + 4);
-  uint64_t* bres_bar = bars + 3 * kMaxStages + 11;   // resident B landed (after the debug slots)
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int bk = args.bk;
-  const int box_bytes = bk * 128;            // one MN-major TMA box: [bk rows][128 B]
-  const int nkb_total = (args.GK + bk - 1) / bk;
+  const int nkb_total = (args.GK + BK - 1) / BK;
   const uint32_t rank = CG2 ? cluster_ctarank() : 0u;
   const int tiles_mn = (CG2 ? (args.m_tiles + 1) / 2 : args.m_tiles) * args.n_tiles;
   const int total_tiles = tiles_mn * args.splits;
@@ -150,7 +137,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       mbar_init(&split[s], CG2 ? 2 * kSplitWarps : kSplitWarps);
       mbar_init(&empty[s], 1);
     }
-    mbar_init(bres_bar, 1);
     for (int i = 0; i < 2; ++i) {
       mbar_init(&acc_full[i], 1);
       mbar_init(&acc_empty[i], (CG2 ? 2 : 1) * kEpiWarps);   // one arrival per epilogue warp
@@ -196,77 +182,38 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // which made the producer the bottleneck of every GEMM with an MN-major operand.
     {
       const uint32_t tx_bytes =
-          args.a_tile_bytes +
-          (b_res ? 0 : args.b_tile_bytes * ((PASSES == 3 && !SPLIT_B) ? 2 : 1));
+          args.a_tile_bytes + args.b_tile_bytes * ((PASSES == 3 && !SPLIT_B) ? 2 : 1);
       const int nA = A_MN ? BM / 32 : 1;
-      const int nB = b_res ? 0 : (B_MN ? args.b_tile_bytes / box_bytes : 1);
-      const int nBlo = (PASSES == 3 && !SPLIT_B && !b_res) ? nB : 0;
-      if (b_res) {
-        // this CTA's half of W^T hi / lo, all k blocks, once: the tiles then stream A only
-        if (lane == 0) mbar_expect_tx(bres_bar, (uint32_t)nkb_all * 2u * args.b_tile_bytes);
-        __syncwarp();
-        for (int l = lane; l < 2 * nkb_all; l += 32) {
-          const int kbi = l >> 1;
-          unsigned char* dst = bres + static_cast<size_t>(kbi) * 2 * args.b_tile_bytes +
-                               (l & 1) * args.b_tile_bytes;
-          tma_load_2d(dst, (l & 1) ? &tmBlo : &tmB, bres_bar, kbi * bk,
-                      (int)rank * (args.n_umma >> 1));
-        }
-      }
+      const int nB = B_MN ? args.b_tile_bytes / kBoxBytes : 1;
+      const int nBlo = (PASSES == 3 && !SPLIT_B) ? nB : 0;
       uint32_t it = 0;
       long long w_empty = 0;
       const long long t_start = clock64();
-      // L2 prefetch cursor: runs args.pf_dist k blocks ahead of the loads (across tiles), so
-      // that the operands streamed from HBM are L2 hits by the time their stage is free.  The
-      // bytes in flight are otherwise bounded by the ring (2-4 stages of 36-80 KB), which at
-      // HBM latency caps a CTA at ~20 B / cycle (profiles/r02_tc_gemm_wait_cycles.txt).
-      int pf_tile = tile0, pf_kb = 0, pf_m0 = 0, pf_n0 = 0, pf_z = 0, pf_kbb = 0, pf_nkb = 0;
-      if (pf_tile < total_tiles) decode(pf_tile, pf_m0, pf_n0, pf_z, pf_kbb, pf_nkb);
-      auto pf_issue = [&]() {
-        while (pf_tile < total_tiles && pf_kb >= pf_nkb) {   // next tile of this CTA
-          pf_tile += tstep;
-          pf_kb = 0;
-          if (pf_tile < total_tiles) decode(pf_tile, pf_m0, pf_n0, pf_z, pf_kbb, pf_nkb);
-        }
-        if (pf_tile >= total_tiles) return;
-        const int k0 = (pf_kbb + pf_kb) * bk;
-        if (lane < nA) {
-          if (!A_MN) tma_prefetch_2d(&tmA, k0, pf_m0);
-          else tma_prefetch_2d(&tmA, pf_m0 + 32 * lane, k0);
-        } else if (SPLIT_B && lane < nA + nB) {   // pre-split B = weights: L2-resident anyway
-          const int j = lane - nA;
-          if (!B_MN) tma_prefetch_2d(&tmB, k0, pf_n0);
-          else tma_prefetch_2d(&tmB, pf_n0 + 32 * j, k0);
-        }
-        ++pf_kb;
-      };
-      for (int i = 0; i < args.pf_dist; ++i) pf_issue();
       for (int tile = tile0; tile < total_tiles; tile += tstep) {
         int m0, n0, z, kb_begin, nkb;
         decode(tile, m0, n0, z, kb_begin, nkb);
         for (int kb = 0; kb < nkb; ++kb, ++it) {
           const int s = it % S;
           const uint32_t ph = (it / S) & 1;
-          if (args.pf_dist > 0) pf_issue();
           w_empty += mbar_wait(&empty[s], ph ^ 1);
           if (lane == 0) mbar_expect_tx(&full[s], tx_bytes);
           __syncwarp();
-          const int k0 = (kb_begin + kb) * bk;
+          const int k0 = (kb_begin + kb) * BK;
           if (lane < nA) {
             if (!A_MN) tma_load_2d(sA_hi(s), &tmA, &full[s], k0, m0);      // box [128 rows][32 k]
-            else tma_load_2d(sA_hi(s) + lane * box_bytes, &tmA, &full[s], m0 + 32 * lane, k0);
+            else tma_load_2d(sA_hi(s) + lane * kBoxBytes, &tmA, &full[s], m0 + 32 * lane, k0);
           } else if (lane < nA + nB) {
             const int j = lane - nA;
             // (pairs: box [N / 2 rows][32 k], this CTA's half of the tile)
             if (!B_MN) tma_load_2d(sB_hi(s), &tmB, &full[s], k0,
                                    n0 + (CG2 ? (int)rank * (args.n_umma >> 1) : 0));
-            else tma_load_2d(sB_hi(s) + j * box_bytes, &tmB, &full[s],
+            else tma_load_2d(sB_hi(s) + j * kBoxBytes, &tmB, &full[s],
                              n0 + (CG2 ? (int)rank * (args.n_umma >> 1) : 0) + 32 * j, k0);
           } else if (lane < nA + nB + nBlo) {
             const int j = lane - nA - nB;
             if (!B_MN) tma_load_2d(sB_lo(s), &tmBlo, &full[s], k0,
                                    n0 + (CG2 ? (int)rank * (args.n_umma >> 1) : 0));
-            else tma_load_2d(sB_lo(s) + j * box_bytes, &tmBlo, &full[s], n0 + 32 * j, k0);
+            else tma_load_2d(sB_lo(s) + j * kBoxBytes, &tmBlo, &full[s], n0 + 32 * j, k0);
           }
         }
       }
@@ -285,9 +232,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                              (static_cast<uint32_t>((CG2 ? 2 * BM : BM) >> 4) << 24);
       const uint32_t a_step = A_MN ? 1024u : 32u;   // bytes per UMMA K step (8 fp32)
       const uint32_t b_step = B_MN ? 1024u : 32u;
-      const uint32_t a_lbo = A_MN ? (uint32_t)box_bytes : 16u;
-      const uint32_t b_lbo = B_MN ? (uint32_t)box_bytes : 16u;
-      const int ksteps_full = bk / 8;
+      const uint32_t a_lbo = A_MN ? (uint32_t)kBoxBytes : 16u;
+      const uint32_t b_lbo = B_MN ? (uint32_t)kBoxBytes : 16u;
       const uint32_t a_sbo = A_MN ? 512u : 1024u, b_sbo = B_MN ? 512u : 1024u;
       const uint32_t a_lt = A_MN ? 1u : 2u, b_lt = B_MN ? 1u : 2u;
       uint32_t it = 0, tcount = 0;
@@ -310,10 +256,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           tc_fence_after();
           if (args.dbg) w_full += clock64() - tw0;
           const uint32_t a_hi = smem_u32(sA_hi(s)), a_lo = smem_u32(sA_lo(s));
-          const uint32_t b_hi =
-              b_res ? smem_u32(bres + static_cast<size_t>(kb_begin + kb) * 2 * args.b_tile_bytes)
-                    : smem_u32(sB_hi(s));
-          const uint32_t b_lo = b_res ? b_hi + args.b_tile_bytes : smem_u32(sB_lo(s));
+          const uint32_t b_hi = smem_u32(sB_hi(s)), b_lo = smem_u32(sB_lo(s));
           // descriptors of the stage once; a k step only adds (bytes >> 4) to the address field
           const uint64_t da_hi0 = make_smem_desc(a_hi, a_lbo, a_sbo, a_lt);
           const uint64_t da_lo0 = make_smem_desc(a_lo, a_lbo, a_sbo, a_lt);
@@ -321,8 +264,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
           const uint64_t db_lo0 = make_smem_desc(b_lo, b_lbo, b_sbo, b_lt);
           // the last k block of a K that is no multiple of 32 holds zeros past K (TMA fill):
           // skip the all-zero k steps
-          const int krem = args.GK - (kb_begin + kb) * bk;
-          const int ksteps = krem >= bk ? ksteps_full : (krem + 7) / 8;
+          const int krem = args.GK - (kb_begin + kb) * BK;
+          const int ksteps = krem >= BK ? BK / 8 : (krem + 7) / 8;
           if (PASSES == 3 && args.a_tmem) {
             // A_hi / A_lo sit in tensor memory (written by the splitters)
             const uint32_t ta_hi = tmem_base + args.a_col0 + static_cast<uint32_t>(s) * 64u;
@@ -384,9 +327,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
       const int b_chunks = SPLIT_B ? args.b_tile_bytes / 16 : 0;
       uint32_t it = 0;
       long long w_tma = 0;
-      // resident B: a splitter's first arrival at the leader also says "my CTA's half of B
-      // has landed" (the leader's MMAs read both halves)
-      if (b_res) mbar_wait(bres_bar, 0);
       for (int tile = tile0; tile < total_tiles; tile += tstep) {
         int m0, n0, z, kb_begin, nkb;
         decode(tile, m0, n0, z, kb_begin, nkb);
@@ -432,7 +372,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             // column = k) is free.  32 B chunks are XOR-ed with (k % 4) by the 32 B-atom
             // swizzle.  Each of the two warps of a quarter takes 16 of the 32 k rows.
             const int q = warp & 3, hsel = (warp - 2) >> 2;
-            const unsigned char* box = sA_hi(s) + q * box_bytes + ((lane & 7) << 2);
+            const unsigned char* box = sA_hi(s) + q * kBoxBytes + ((lane & 7) << 2);
             const int c32 = lane >> 3;
             uint32_t h[16], l[16];
 #pragma unroll
@@ -875,47 +815,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 }
 
 // ------------------------------------------------------------------ host -------
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
-                             const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                             const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeFn get_encode_fn() {
-  static EncodeFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) !=
-          cudaSuccess ||
-      qres != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<EncodeFn>(p);
-  return fn;
-}
-
-// 2D fp32 tensor [outer rows][inner cols], box [box_outer][32 cols], 128B swizzle.
+// 2D fp32 tensor [outer rows][inner cols], box [box_outer][32 cols], 128B swizzle (the 32 B
+// atom variant for MN-major operands).
 static int encode_2d(CUtensorMap* tm, const float* ptr, uint64_t inner, uint64_t outer,
                      uint64_t ld_floats, uint32_t box_outer, bool mn_major) {
-  EncodeFn fn = get_encode_fn();
-  if (!fn) {
-    set_error("cuTensorMapEncodeTiled is not available from the CUDA driver");
-    return TFR_CUDA_ERROR;
-  }
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld_floats * sizeof(float)};
-  cuuint32_t box[2] = {BK, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<float*>(ptr), dims, strides,
-                  box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                  mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (ptr %p inner %llu outer %llu ld %llu "
-              "box_outer %u)", (int)r, (const void*)ptr, (unsigned long long)inner,
-              (unsigned long long)outer, (unsigned long long)ld_floats, box_outer);
-    return TFR_CUDA_ERROR;
-  }
-  return TFR_OK;
+  return encode_tmap_2d(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, ptr, inner, outer,
+                        ld_floats * sizeof(float), BK, box_outer,
+                        mn_major ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 bool shape_supported(int lda, int ldb) { return lda % 4 == 0 && ldb % 4 == 0; }
@@ -971,111 +877,79 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   TFR_REQUIRE(!pre_split_b || (reinterpret_cast<uintptr_t>(g.B_lo) & 15) == 0, "tc gemm: B_lo alignment");
 
   // N tiling: one tile if it fits a single UMMA (N <= 256), else tiles of 256.
-  static const int n_cap = getenv("TFR_TC_NCAP") ? atoi(getenv("TFR_TC_NCAP")) : 256;
-  static const bool no_pairs = getenv("TFR_TC_NO_PAIRS") != nullptr;
-  static const bool no_pairs_mn = getenv("TFR_TC_NO_PAIRS_MN") != nullptr;
   // dW GEMMs as CTA pairs: each CTA stages its 128 rows of the M side and HALF of the N side
   // (whole 32-column boxes), so N is rounded up to a multiple of 64.
-  const bool want_pairs_mn = !no_pairs && !no_pairs_mn && g.passes == 3 && g.a_mn && g.b_mn &&
-                             g.split_b && g.GM > BM && (g.GN + 63) / 64 * 64 <= n_cap;
+  const bool want_pairs_mn = g.passes == 3 && g.a_mn && g.b_mn && g.split_b && g.GM > BM &&
+                             (g.GN + 63) / 64 * 64 <= kMaxN;
   const int n_umma = want_pairs_mn ? (g.GN + 63) / 64 * 64
-                                   : (g.GN <= n_cap ? ((g.GN + 15) / 16) * 16 : n_cap);
+                                   : (g.GN <= kMaxN ? ((g.GN + 15) / 16) * 16 : kMaxN);
   const int n_tiles = (g.GN + n_umma - 1) / n_umma;
-  // Stage depth in k: the 128 B swizzle pins K-major tiles to 32 fp32 of k; MN-major tiles
-  // may use 16 k-rows, which halves the stage and doubles the ring depth (the dW GEMMs
-  // stream both operands from HBM and are latency-bound with 2-3 stages).
-  const int bk = 32;   // (16-row MN-major stages were measured slower: more TMA boxes per byte)
-  const int a_tile_bytes = g.a_mn ? (BM / 32) * bk * 128 : kATileBytes;
-  int b_tile_bytes = g.b_mn ? ((n_umma + 31) / 32) * bk * 128 : n_umma * 128;
+  // Stage depth in k is BK for both majornesses (16-row MN-major stages, which would deepen
+  // the ring of the dW GEMMs, were measured slower: more TMA boxes per byte).
+  const int a_tile_bytes = g.a_mn ? (BM / 32) * kBoxBytes : kATileBytes;
+  int b_tile_bytes = g.b_mn ? ((n_umma + 31) / 32) * kBoxBytes : n_umma * 128;
   const int copies = g.passes == 3 ? 2 : 1;
   uint32_t acc_cols = 32;
   while ((int)acc_cols < n_umma) acc_cols <<= 1;
   // A in tensor memory: needs 64 columns per stage next to the two accumulators
-  static const bool no_a_tmem = getenv("TFR_TC_NO_A_TMEM") != nullptr;
   // (K-major A with pre-split B: forward / dZ GEMMs.  MN-major A with B split on the fly: the
   //  dW GEMMs, whose tiles are long split-K loops — one accumulator buffer is enough there,
   //  which leaves the columns for the A stages even at N = 256.)
-  static const bool no_a_tmem_mn = getenv("TFR_TC_NO_A_TMEM_MN") != nullptr;
   const bool a_tmem_k = !g.a_mn && !g.split_b;
-  const bool a_tmem_mn = g.a_mn && g.split_b && !no_a_tmem_mn;
+  const bool a_tmem_mn = g.a_mn && g.split_b;
   uint32_t acc_bufs = 2;
   if (a_tmem_mn && 2 * acc_cols + 3 * 64 > 512) acc_bufs = 1;
-  bool a_tmem = !no_a_tmem && g.passes == 3 && (a_tmem_k || a_tmem_mn) &&
-                acc_bufs * acc_cols + 2 * 64 <= 512;
+  bool a_tmem = g.passes == 3 && (a_tmem_k || a_tmem_mn) && acc_bufs * acc_cols + 2 * 64 <= 512;
   if (!a_tmem) acc_bufs = 2;
   // CTA pairs (see the kernel's CG2 note): forward / dZ GEMMs with one n tile.
   const int m_tiles_all = (g.GM + BM - 1) / BM;
-  const bool cg2_k = !no_pairs && g.passes == 3 && a_tmem_k && !g.b_mn && n_tiles == 1 &&
-                     (g.splits <= 1) && n_umma % 32 == 0 && m_tiles_all >= 4;
+  const bool cg2_k = g.passes == 3 && a_tmem_k && !g.b_mn && n_tiles == 1 && (g.splits <= 1) &&
+                     n_umma % 32 == 0 && m_tiles_all >= 4;
   const bool cg2_mn = want_pairs_mn && a_tmem && n_tiles == 1;
   const bool cg2 = cg2_k || cg2_mn;
-  if (cg2_k) b_tile_bytes = (n_umma / 2) * 128;          // this CTA's half of the B tile
-  if (cg2_mn) b_tile_bytes = (n_umma / 64) * bk * 128;   // ... as whole [32 k][32 n] boxes
-  int stage_bytes = a_tmem ? a_tile_bytes + b_tile_bytes * copies
-                           : (a_tile_bytes + b_tile_bytes) * copies;
-  // Resident B (pairs, pre-split K-major weights): if this CTA's half of W^T hi + lo over the
-  // whole K fits next to >= 2 A stages, it is loaded once per CTA instead of once per tile —
-  // the weights were 50-80 % of the bytes these GEMMs pull through TMA.
-  // Measured at config 2 (profiles/README.md, round 2): NO gain — 0.693-0.705 ms/step with
-  // resident weights (L2, L3, dZ2; dZ1 with 2 stages) against 0.686 without: the weight tiles
-  // are L2 hits shared by all CTAs and were not what bounds these GEMMs any more.  Opt-in.
-  static const bool no_b_resident = getenv("TFR_TC_B_RESIDENT") == nullptr;
-  const size_t b_res_bytes = (size_t)((g.GK + bk - 1) / bk) * 2 * b_tile_bytes;
-  const int a_stage_bytes = a_tmem ? a_tile_bytes : a_tile_bytes * copies;
-  bool b_resident = false;
-  static const int bres_min_stages =
-      getenv("TFR_TC_BRES_MIN_STAGES") ? atoi(getenv("TFR_TC_BRES_MIN_STAGES")) : 2;
-  if (cg2_k && !no_b_resident &&
-      b_res_bytes + (size_t)bres_min_stages * a_stage_bytes + 35 * 1024 <= 227 * 1024) {
-    b_resident = true;
-    stage_bytes = a_stage_bytes;
-  }
+  if (cg2_k) b_tile_bytes = (n_umma / 2) * 128;         // this CTA's half of the B tile
+  if (cg2_mn) b_tile_bytes = (n_umma / 64) * kBoxBytes; // ... as whole [32 k][32 n] boxes
+  const int stage_bytes = a_tmem ? a_tile_bytes + b_tile_bytes * copies
+                                 : (a_tile_bytes + b_tile_bytes) * copies;
   int splits = g.splits < 1 ? 1 : g.splits;
   // TMA-store epilogue: row-major, unsplit output with 16-byte aligned rows.
-  static const bool no_tma_store = getenv("TFR_TC_NO_TMA_STORE") != nullptr;
   const bool tma_store =
-      !no_tma_store && g.epi != EPI_MASK_POS && !g.store_transposed && splits == 1 &&
+      g.epi != EPI_MASK_POS && !g.store_transposed && splits == 1 &&
       g.ldc % 4 == 0 && g.GN % 4 == 0 && (reinterpret_cast<uintptr_t>(g.C) & 15) == 0 &&
       (!g.bias || (reinterpret_cast<uintptr_t>(g.bias) & 15) == 0) &&
       (n_tiles == 1 || n_umma % 32 == 0);
   const bool colsum_regs = tma_store && g.colsum && n_tiles == 1;
   const int colsum_cols = (g.colsum && !colsum_regs) ? ((g.GN + 3) / 4) * 4 : 0;
   TFR_REQUIRE(colsum_cols <= 1024, "tc gemm: colsum output supports GN <= 1024");
-  // Two staging tiles per epilogue warp when that does not cost a pipeline stage.
   const int bias_cols = (tma_store && g.epi == EPI_BIAS_ACT) ? ((n_tiles * n_umma + 31) / 32) * 32 : 0;
   const size_t fixed1 = kEpiSmemBytes + kEpiWarps * colsum_cols * sizeof(float);
   const size_t fixed2 = kEpiSmemBytes2 + (kEpiWarps * colsum_cols + bias_cols) * sizeof(float);
   const size_t budget = 227 * 1024 - 1024 /*align*/ - 256 /*barriers*/;
   const int epi_smem_bytes = tma_store ? kEpiSmemBytes2 : kEpiSmemBytes;
-  const size_t resident = b_resident ? b_res_bytes : 0;
-  if (b_resident && budget < (tma_store ? fixed2 : fixed1) + resident + 2 * (size_t)stage_bytes) {
-    set_error("tc gemm: internal: resident B does not fit");   // (excluded by the test above)
-    return TFR_UNSUPPORTED;
-  }
-  int stages = (int)((budget - (tma_store ? fixed2 : fixed1) - resident) / stage_bytes);
+  int stages = (int)((budget - (tma_store ? fixed2 : fixed1)) / stage_bytes);
   if (stages > kMaxStages) stages = kMaxStages;
   if (a_tmem) {
     const int room = (512 - (int)(acc_bufs * acc_cols)) / 64;   // A stages that fit tensor memory
     if (stages > room) stages = room;
   }
   TFR_REQUIRE(stages >= 1, "tc gemm: tile does not fit shared memory");
-  const int nkb_total = (g.GK + bk - 1) / bk;
+  const int nkb_total = (g.GK + BK - 1) / BK;
   int kb_per_split = (nkb_total + splits - 1) / splits;
   // (a split whose k range is empty stores zeros, so any split count is legal)
 
   CUtensorMap tmA, tmB, tmBlo;
   int rc;
   if (!g.a_mn) rc = encode_2d(&tmA, g.A, (uint64_t)g.GK, (uint64_t)g.GM, (uint64_t)g.lda, BM, false);
-  else rc = encode_2d(&tmA, g.A, (uint64_t)g.GM, (uint64_t)g.GK, (uint64_t)g.lda, (uint32_t)bk, true);
+  else rc = encode_2d(&tmA, g.A, (uint64_t)g.GM, (uint64_t)g.GK, (uint64_t)g.lda, (uint32_t)BK, true);
   if (rc) return rc;
   const uint32_t b_box_rows = cg2 ? (uint32_t)n_umma / 2 : (uint32_t)n_umma;
   if (!g.b_mn) rc = encode_2d(&tmB, g.B, (uint64_t)g.GK, (uint64_t)g.GN, (uint64_t)g.ldb, b_box_rows, false);
-  else rc = encode_2d(&tmB, g.B, (uint64_t)g.GN, (uint64_t)g.GK, (uint64_t)g.ldb, (uint32_t)bk, true);
+  else rc = encode_2d(&tmB, g.B, (uint64_t)g.GN, (uint64_t)g.GK, (uint64_t)g.ldb, (uint32_t)BK, true);
   if (rc) return rc;
   tmBlo = tmB;
   if (pre_split_b) {
     if (!g.b_mn) rc = encode_2d(&tmBlo, g.B_lo, (uint64_t)g.GK, (uint64_t)g.GN, (uint64_t)g.ldb, b_box_rows, false);
-    else rc = encode_2d(&tmBlo, g.B_lo, (uint64_t)g.GN, (uint64_t)g.GK, (uint64_t)g.ldb, (uint32_t)bk, true);
+    else rc = encode_2d(&tmBlo, g.B_lo, (uint64_t)g.GN, (uint64_t)g.GK, (uint64_t)g.ldb, (uint32_t)BK, true);
     if (rc) return rc;
   }
 
@@ -1084,7 +958,6 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   ka.GM = g.GM; ka.GN = g.GN; ka.GK = g.GK;
   ka.n_umma = n_umma;
   ka.b_tile_bytes = b_tile_bytes;
-  ka.bk = bk;
   ka.a_tile_bytes = a_tile_bytes;
   ka.stages = stages;
   ka.epi = g.epi; ka.act = g.act; ka.store_transposed = g.store_transposed;
@@ -1094,14 +967,6 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   ka.tmem_cols = acc_cols;     // per accumulator buffer; the kernel allocates two
   ka.a_tmem = a_tmem ? 1 : 0;
   ka.acc_bufs = acc_bufs;
-  ka.b_resident = b_resident ? 1 : 0;
-  {
-    static const int pf_env = getenv("TFR_TC_PREFETCH") ? atoi(getenv("TFR_TC_PREFETCH")) : -1;
-    // Measured (profiles/README.md, round 2): prefetching ahead LOSES 3-5 % on the dW GEMMs —
-    // these kernels are bound by the chip-wide TMA load rate (~6.3 TB/s), not by latency,
-    // so the extra requests only compete with the loads.  Off unless asked for.
-    ka.pf_dist = pf_env >= 0 ? pf_env : 0;
-  }
   ka.a_col0 = acc_bufs * acc_cols;
   {
     uint32_t need = acc_bufs * acc_cols + (a_tmem ? 64u * (uint32_t)stages : 0u), alloc = 32;
@@ -1123,7 +988,6 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   TFR_REQUIRE(g.epi != EPI_BIAS_ACT || g.bias, "tc gemm: bias required");
   TFR_REQUIRE(g.epi != EPI_MASK_POS || g.aux, "tc gemm: aux required");
   ka.tma_store = tma_store;
-  ka.epi_bufs = 1;
   ka.epi_smem_bytes = epi_smem_bytes;
   ka.colsum_regs = colsum_regs;
   ka.bias_cols = bias_cols;
@@ -1142,48 +1006,39 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   ka.n_tiles = n_tiles;
   ka.splits = splits;
   const int total_tiles = ka.m_tiles * ka.n_tiles * splits;
-  static int num_sms = 0;
-  if (num_sms == 0) {
-    int dev = 0;
-    TFR_CUDA_OK(cudaGetDevice(&dev));
-    TFR_CUDA_OK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
-  dim3 grid(total_tiles < num_sms ? total_tiles : num_sms);
+  const int sms = num_sms();
+  dim3 grid(total_tiles < sms ? total_tiles : sms);
   if (cg2) {
     const int pair_tiles = (ka.m_tiles + 1) / 2 * ka.n_tiles * splits;
-    const int pairs = pair_tiles < num_sms / 2 ? pair_tiles : num_sms / 2;
+    const int pairs = pair_tiles < sms / 2 ? pair_tiles : sms / 2;
     grid = dim3(2 * pairs);
   }
-  const size_t smem = (size_t)stages * stage_bytes + resident + epi_smem_bytes +
+  const size_t smem = (size_t)stages * stage_bytes + epi_smem_bytes +
                       (kEpiWarps * colsum_cols + bias_cols) * sizeof(float) + 1024 /*align*/ +
                       256 /*barriers*/;
   if (g.colsum_slots_out) *g.colsum_slots_out = kEpiWarps * (int)grid.x;
 
   if (cg2) {
-    static const bool no_fast_epi = getenv("TFR_TC_NO_FAST_EPI") != nullptr;
     if (cg2_mn) {
-      if (!no_fast_epi && !ka.tma_store && g.epi == EPI_STORE)
+      if (!ka.tma_store && g.epi == EPI_STORE)
         return launch_pairs<true, 4>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st);
       return launch_pairs<true, -1>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st);
     }
-    if (!no_fast_epi && ka.tma_store && g.epi == EPI_STORE)
+    if (ka.tma_store && g.epi == EPI_STORE)
       return launch_pairs<false, 0>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st);
-    if (!no_fast_epi && ka.tma_store && g.epi == EPI_BIAS_ACT && g.act == TFR_ACT_RELU)
+    if (ka.tma_store && g.epi == EPI_BIAS_ACT && g.act == TFR_ACT_RELU)
       return launch_pairs<false, 1>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st);
-    if (!no_fast_epi && ka.tma_store && g.epi == EPI_MASK_BITS)
+    if (ka.tma_store && g.epi == EPI_MASK_BITS)
       return launch_pairs<false, 3>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st);
     return launch_pairs<false, -1>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st);
   }
-  {
-    static const bool no_fast_epi = getenv("TFR_TC_NO_FAST_EPI") != nullptr;
-    if (!no_fast_epi && g.a_mn && g.b_mn && g.passes == 3 && g.split_b && !ka.tma_store &&
-        g.epi == EPI_STORE) {   // single-CTA dW GEMM (one 128-row block): plain-store kernel
-      auto kern = tc_gemm_kernel<true, true, 3, true, false, 4>;
-      TFR_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      kern<<<grid, kThreads, smem, st>>>(tmA, tmB, tmBlo, tmC, ka);
-      TFR_LAUNCH_OK();
-      return TFR_OK;
-    }
+  if (g.a_mn && g.b_mn && g.passes == 3 && g.split_b && !ka.tma_store &&
+      g.epi == EPI_STORE) {   // single-CTA dW GEMM (one 128-row block): plain-store kernel
+    auto kern = tc_gemm_kernel<true, true, 3, true, false, 4>;
+    TFR_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<grid, kThreads, smem, st>>>(tmA, tmB, tmBlo, tmC, ka);
+    TFR_LAUNCH_OK();
+    return TFR_OK;
   }
 #define TFR_TC_LAUNCH(AMN, BMN, P, SB) \
   return launch<AMN, BMN, P, SB>(tmA, tmB, tmBlo, tmC, ka, grid, smem, st)

@@ -22,10 +22,9 @@
 #include <cuda.h>
 #include <cuda_bf16.h>
 
-#include <cstdlib>
-
 #include "common.cuh"
 #include "tc_gemm_bf16.cuh"
+#include "tc_host.h"
 #include "tc_ptx.cuh"
 
 namespace tfr {
@@ -48,17 +47,6 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       "elect.sync _|q, 0xffffffff;\n\t"
       "setp.ne.b32 p, %4, 0;\n\t"
       "@q tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-__device__ __forceinline__ void umma_bf16_cg2(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
-                                              uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\t"
-      "elect.sync _|q, 0xffffffff;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "@q tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
@@ -102,13 +90,7 @@ struct KArgs {
   int c_rows_per_split;
 };
 
-// CG2 (K-major layout only): CTA pairs, tcgen05 cta_group::2 — the pair owns 256 rows, each
-// CTA stages its 128 rows of A and HALF of the B tile (N / 2 rows of W), which cuts the bytes
-// a CTA loads per k block from 16 + N / 8 to 16 + N / 16 KB (these GEMMs run at the chip-wide
-// TMA load rate, DESIGN.md §3).  The peer's idle MMA warp relays "my stage has landed" to the
-// leader's `peer` barriers; the leader issues the M = 256 MMAs and releases stages /
-// publishes accumulators in both CTAs with multicast commits.
-template <bool MN, bool CG2 = false>
+template <bool MN>
 __global__ void __launch_bounds__(kThreads, 1)
 bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                  const __grid_constant__ CUtensorMap tmC, const KArgs args) {
@@ -126,15 +108,13 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   uint64_t* empty = bars + kMaxStages;
   uint64_t* acc_full = bars + 2 * kMaxStages;
   uint64_t* acc_empty = bars + 2 * kMaxStages + 2;
-  uint64_t* peer = bars + 2 * kMaxStages + 4;     // [kMaxStages] pairs: the peer's stage landed
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 3 * kMaxStages + 4);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kMaxStages + 4);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = CG2 ? cluster_ctarank() : 0u;
-  const int items_per_z = (CG2 ? (args.m_groups + 1) / 2 : args.m_groups) * args.n_tiles;
+  const int items_per_z = args.m_groups * args.n_tiles;
   const int total_items = items_per_z * args.splits;
-  const int item0 = CG2 ? (int)(blockIdx.x >> 1) : (int)blockIdx.x;
-  const int istep = CG2 ? (int)(gridDim.x >> 1) : (int)gridDim.x;
+  const int item0 = (int)blockIdx.x;
+  const int istep = (int)gridDim.x;
 
   if (threadIdx.x == 0) {
     prefetch_tmap(&tmA);
@@ -143,26 +123,19 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     for (int s = 0; s < S; ++s) {
       mbar_init(&full[s], 1);
       mbar_init(&empty[s], 1);
-      mbar_init(&peer[s], 1);
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&acc_full[i], 1);
-      mbar_init(&acc_empty[i], (CG2 ? 2 : 1) * kEpiWarps);   // one arrival per epilogue warp
+      mbar_init(&acc_empty[i], kEpiWarps);   // one arrival per epilogue warp
     }
     fence_barrier_init();
   }
   if (warp == 1) {
-    if (CG2) {
-      tmem_alloc2(tmem_slot, args.tmem_alloc_cols);
-      tmem_relinquish2();
-    } else {
-      tmem_alloc(tmem_slot, args.tmem_alloc_cols);
-      tmem_relinquish();
-    }
+    tmem_alloc(tmem_slot, args.tmem_alloc_cols);
+    tmem_relinquish();
   }
   tc_fence_before();
   __syncthreads();
-  if (CG2) cluster_sync_all();
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
@@ -171,7 +144,7 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   auto decode = [&](int item, int& m0, int& n0, int& z, int& kb_begin, int& nkb) {
     z = item / items_per_z;
     const int r = item - z * items_per_z;
-    m0 = CG2 ? (r / args.n_tiles) * 2 * BM + (int)rank * BM : (r / args.n_tiles) * MT * BM;
+    m0 = (r / args.n_tiles) * MT * BM;
     n0 = (r % args.n_tiles) * args.n_umma;
     kb_begin = z * args.kb_per_split;
     const int kb_end = min(args.nkb_total, kb_begin + args.kb_per_split);
@@ -202,26 +175,10 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             else tma_load_2d(sA(s) + lane * 8192, &tmA, &full[s], m0 + 64 * lane, k0);   // {64 m, 64 k}
           } else if (lane < nA + nB) {
             const int j = lane - nA;
-            // box {64 k, n_umma rows}; pairs: {64 k, n_umma / 2 rows}, this CTA's half
-            if (!MN) tma_load_2d(sB(s), &tmB, &full[s], k0,
-                                 n0 + (CG2 ? (int)rank * (args.n_umma >> 1) : 0));
+            if (!MN) tma_load_2d(sB(s), &tmB, &full[s], k0, n0);     // box {64 k, n_umma rows}
             else tma_load_2d(sB(s) + j * 8192, &tmB, &full[s], n0 + 64 * j, k0);         // {64 n, 64 k}
           }
         }
-      }
-    }
-  } else if (warp == 1 && CG2 && rank != 0) {
-    // ------------------------------------ the peer's relay (its MMA warp is idle) ----
-    const uint32_t leader_peer0 = mapa_u32(&peer[0], 0);
-    uint32_t it = 0;
-    for (int item = item0; item < total_items; item += istep) {
-      int m0, n0, z, kb_begin, nkb;
-      decode(item, m0, n0, z, kb_begin, nkb);
-      for (int kb = 0; kb < nkb; ++kb, ++it) {
-        const int s = it % S;
-        mbar_wait(&full[s], (it / S) & 1);
-        if (lane == 0) mbar_arrive_cluster(leader_peer0 + (uint32_t)s * 8u);
-        __syncwarp();
       }
     }
   } else if (warp == 1) {
@@ -230,7 +187,7 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     const uint32_t idesc = (1u << 4) | (1u << 7) | (1u << 10) |
                            (static_cast<uint32_t>(MN) << 15) | (static_cast<uint32_t>(MN) << 16) |
                            (static_cast<uint32_t>(args.n_umma >> 3) << 17) |
-                           (static_cast<uint32_t>((CG2 ? 2 * BM : BM) >> 4) << 24);
+                           (static_cast<uint32_t>(BM >> 4) << 24);
     // K-major: 128 B rows, 8-row atoms every 1024 B, a k step (16 bf16) = 32 B.
     // MN-major: rows = k (128 B = 64 m / n), 8-k atoms every 1024 B, the next 64 m / n at
     // LBO = 8192 B (the next TMA box), a k step (16 rows) = 2048 B.
@@ -248,7 +205,6 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
         const int s = it % S;
         const uint32_t ph = (it / S) & 1;
         mbar_wait(&full[s], ph);
-        if (CG2) mbar_wait(&peer[s], ph);   // ... and the peer's half of the stage
         tc_fence_after();
         const int krem = args.GK - (kb_begin + kb) * BK;
         const int ksteps = krem >= BK ? BK / 16 : (krem + 15) / 16;
@@ -257,21 +213,13 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
           const uint64_t da0 = make_smem_desc(smem_u32(sA(s) + mt * kATileBytes), lbo, sbo, 2u);
           const uint32_t tmem_d = tmem_d0 + mt * args.acc_cols;
 #pragma unroll 4
-          for (int ks = 0; ks < ksteps; ++ks) {
-            if (CG2)
-              umma_bf16_cg2(tmem_d, da0 + static_cast<uint64_t>(ks * step16),
-                            db0 + static_cast<uint64_t>(ks * step16), idesc,
-                            (kb | ks) != 0 ? 1u : 0u);
-            else
-              umma_bf16(tmem_d, da0 + static_cast<uint64_t>(ks * step16),
-                        db0 + static_cast<uint64_t>(ks * step16), idesc, (kb | ks) != 0 ? 1u : 0u);
-          }
+          for (int ks = 0; ks < ksteps; ++ks)
+            umma_bf16(tmem_d, da0 + static_cast<uint64_t>(ks * step16),
+                      db0 + static_cast<uint64_t>(ks * step16), idesc, (kb | ks) != 0 ? 1u : 0u);
         }
-        if (CG2) umma_commit_cg2(&empty[s]);
-        else umma_commit(&empty[s]);
+        umma_commit(&empty[s]);
       }
-      if (CG2) umma_commit_cg2(&acc_full[ab]);
-      else if (nkb > 0) umma_commit(&acc_full[ab]);
+      if (nkb > 0) umma_commit(&acc_full[ab]);
       else if (lane == 0) mbar_arrive(&acc_full[ab]);
       __syncwarp();
     }
@@ -279,14 +227,10 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
     // ---------------------------------------------------- epilogue (warps 2..9)
     const int q = warp & 3;           // TMEM lane quarter this warp may access
     const int ew = warp - 2;          // 0..7
-    // "accumulator drained" (all lanes call it at a warp-uniform point; one lane arrives,
-    // at the MMA issuer's barrier — the leader's in a pair)
+    // "accumulator drained" (all lanes call it at a warp-uniform point; one lane arrives)
     auto arrive_acc_empty = [&](uint32_t ab) {
       __syncwarp();
-      if (lane == 0) {
-        if (CG2) mbar_arrive_cluster(mapa_u32(&acc_empty[ab], 0));
-        else mbar_arrive(&acc_empty[ab]);
-      }
+      if (lane == 0) mbar_arrive(&acc_empty[ab]);
     };
     const int half = ew >> 2;         // which of the two warps of the quarter
     unsigned char* stg = epi_smem + ew * kStagingBytes;
@@ -492,56 +436,17 @@ bf16_gemm_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
   }
   tc_fence_before();
   __syncthreads();
-  if (CG2) cluster_sync_all();
-  if (warp == 1) {
-    if (CG2) tmem_dealloc2(tmem_base, args.tmem_alloc_cols);
-    else tmem_dealloc(tmem_base, args.tmem_alloc_cols);
-  }
+  if (warp == 1) tmem_dealloc(tmem_base, args.tmem_alloc_cols);
 }
 
 // ------------------------------------------------------------------ host -------
-typedef CUresult (*EncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
-                             const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                             const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                             CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static EncodeFn get_encode_fn() {
-  static EncodeFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult qres;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) !=
-          cudaSuccess ||
-      qres != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<EncodeFn>(p);
-  return fn;
-}
-
-// 2D tensor [outer rows][inner cols] of `esize`-byte elements, 128B swizzle, box
-// {box_inner (= 128 B), box_outer}.
+// 2D tensor [outer rows][inner cols] of `esize`-byte elements (bf16 or fp32), 128B swizzle,
+// box {box_inner (= 128 B), box_outer}.
 static int encode_2d(CUtensorMap* tm, const void* ptr, int esize, uint64_t inner, uint64_t outer,
                      uint64_t ld_elems, uint32_t box_inner, uint32_t box_outer) {
-  EncodeFn fn = get_encode_fn();
-  if (!fn) {
-    set_error("cuTensorMapEncodeTiled is not available from the CUDA driver");
-    return TFR_CUDA_ERROR;
-  }
-  cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld_elems * (uint64_t)esize};
-  cuuint32_t box[2] = {box_inner, box_outer};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(tm, esize == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32,
-                  2, const_cast<void*>(ptr), dims, strides, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled failed with CUresult %d (ptr %p esize %d inner %llu outer "
-              "%llu ld %llu box %u x %u)", (int)r, ptr, esize, (unsigned long long)inner,
-              (unsigned long long)outer, (unsigned long long)ld_elems, box_inner, box_outer);
-    return TFR_CUDA_ERROR;
-  }
-  return TFR_OK;
+  return encode_tmap_2d(
+      tm, esize == 2 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, ptr,
+      inner, outer, ld_elems * (uint64_t)esize, box_inner, box_outer, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
 template <bool MN>
@@ -550,27 +455,6 @@ static int launch(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensor
   auto kern = bf16_gemm_kernel<MN>;
   TFR_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, kThreads, smem, st>>>(tmA, tmB, tmC, ka);
-  TFR_LAUNCH_OK();
-  return TFR_OK;
-}
-
-static int launch_pairs(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC,
-                        const KArgs& ka, dim3 grid, size_t smem, cudaStream_t st) {
-  auto kern = bf16_gemm_kernel<false, true>;
-  TFR_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2;
-  at[0].val.clusterDim.y = 1;
-  at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  TFR_CUDA_OK(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, tmC, ka));
   TFR_LAUNCH_OK();
   return TFR_OK;
 }
@@ -615,14 +499,7 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   }
   ka.nkb_total = (g.GK + BK - 1) / BK;
   ka.kb_per_split = (ka.nkb_total + ka.splits - 1) / ka.splits;
-  // Measured at config 3 (profiles/README.md, round 2): pairs are 2-12 % SLOWER on the bf16
-  // forward / dZ GEMMs (57 / 39 / 25 / 36 / 58 us without, 58 / 45 / 28 / 39 / 62 us with) — at
-  // half the bytes per element these GEMMs are not bound by the TMA load rate, and the relay
-  // adds a cross-SM hop to every stage.  Opt-in only.
-  static const bool want_pairs = getenv("TFR_BF16_PAIRS") != nullptr;
-  const bool cg2 = want_pairs && !mn && ka.n_tiles == 1 && ka.n_umma % 32 == 0 && ka.m_tiles >= 4;
-  ka.b_tile_bytes = mn ? ((ka.n_umma + 63) / 64) * 8192 : (cg2 ? ka.n_umma / 2 : ka.n_umma) * 128;
-  if (cg2) ka.tmem_alloc_cols = 512;   // all of it: the same base in both CTAs
+  ka.b_tile_bytes = mn ? ((ka.n_umma + 63) / 64) * 8192 : ka.n_umma * 128;
   ka.epi = g.epi; ka.act = g.act; ka.bias = g.bias;
   ka.bias_cols = g.epi == EPI_BIAS_ACT ? ((ka.n_tiles * ka.n_umma + 63) / 64) * 64 + 64 : 0;
   ka.bits_out = g.mask_bits_out; ka.bits_in = g.mask_bits_in;
@@ -651,7 +528,7 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
     rc = encode_2d(&tmA, g.A, 2, (uint64_t)g.GK, (uint64_t)g.GM, (uint64_t)g.lda, BK, BM);
     if (rc) return rc;
     rc = encode_2d(&tmB, g.B, 2, (uint64_t)g.GK, (uint64_t)g.GN, (uint64_t)g.ldb, BK,
-                   (uint32_t)(cg2 ? ka.n_umma / 2 : ka.n_umma));
+                   (uint32_t)ka.n_umma);
     if (rc) return rc;
     rc = encode_2d(&tmC, g.C, 2, (uint64_t)g.GN, (uint64_t)g.GM, (uint64_t)g.ldc, 64, 32);
     if (rc) return rc;
@@ -666,21 +543,10 @@ int gemm(const GemmDesc& g, cudaStream_t st) {
   }
 
   const int total_items = ka.m_groups * ka.n_tiles * ka.splits;
-  static int num_sms = 0;
-  if (num_sms == 0) {
-    int dev = 0;
-    TFR_CUDA_OK(cudaGetDevice(&dev));
-    TFR_CUDA_OK(cudaDeviceGetAttribute(&num_sms, cudaDevAttrMultiProcessorCount, dev));
-  }
-  dim3 grid(total_items < num_sms ? total_items : num_sms);
-  if (cg2) {
-    const int pair_items = (ka.m_groups + 1) / 2 * ka.n_tiles * ka.splits;
-    const int pairs = pair_items < num_sms / 2 ? pair_items : num_sms / 2;
-    grid = dim3(2 * pairs);
-  }
+  const int sms = num_sms();
+  dim3 grid(total_items < sms ? total_items : sms);
   const size_t smem = (size_t)stages * stage_bytes + fixed;
   if (g.colsum_slots_out) *g.colsum_slots_out = kEpiWarps * (int)grid.x;
-  if (cg2) return launch_pairs(tmA, tmB, tmC, ka, grid, smem, st);
   return mn ? launch<true>(tmA, tmB, tmC, ka, grid, smem, st)
             : launch<false>(tmA, tmB, tmC, ka, grid, smem, st);
 }

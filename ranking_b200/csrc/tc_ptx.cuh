@@ -69,14 +69,6 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* tm, ui
       "l"(reinterpret_cast<uint64_t>(tm)), "r"(smem_u32(bar)), "r"(c0), "r"(c1)
       : "memory");
 }
-// Prefetch of a tile into L2 (no shared memory, no barrier): lets a producer run further
-// ahead of the TMA loads than its shared-memory ring is deep.
-__device__ __forceinline__ void tma_prefetch_2d(const CUtensorMap* tm, int c0, int c1) {
-  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(
-                   reinterpret_cast<uint64_t>(tm)),
-               "r"(c0), "r"(c1)
-               : "memory");
-}
 // smem -> global tile store through the async proxy (bulk async-group completion)
 __device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, const void* src, int c0,
                                              int c1) {

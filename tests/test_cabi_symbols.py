@@ -58,3 +58,14 @@ def test_product_has_no_oracle_import():
       if f.endswith('.py'):
         src = open(os.path.join(dirpath, f)).read()
         assert not re.search(r'^\s*(from|import)\s+oracle\b', src, flags=re.M), f
+
+
+def test_native_code_reads_no_environment():
+  """Which kernel runs follows from shapes and arguments only: an environment variable
+  must not switch a library call to another code path."""
+  csrc = os.path.join(ROOT, 'ranking_b200', 'csrc')
+  sources = sorted(f for f in os.listdir(csrc) if f.endswith(('.cu', '.cuh', '.h')))
+  assert any(f.endswith('.cu') for f in sources), sources
+  for f in sources:
+    src = open(os.path.join(csrc, f)).read()
+    assert not re.search(r'getenv\s*\(', src), f
